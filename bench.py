@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200-native large-steps hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload plane1000|...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload plane1000|...] [--dump-outputs DIR]
 
 metric   : from_differential solves/sec @ 1M verts  (BASELINE.json)
 step     : one from_differential solve of a (V,3) right-hand side (forward solve of the optimisation step)
@@ -204,8 +204,11 @@ def run_reference(args, wl, wl_name):
         step(i)
     t0 = time.perf_counter()
     for i in range(args.steps):
-        step(i)
+        x_last = step(i)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "solution.npy"), np.asarray(x_last, dtype=np.float32))
     val_sps = args.steps / dt
     cores = cg.threads if use_cg else 1
     sample = (f"{args.steps} solves of a (V,3) fp32 RHS at V={V} with the faster of two CPU ports of the reference: "
@@ -294,12 +297,16 @@ def run_b200(args, wl, wl_name):
 
     # ---- value: device-resident right-hand sides ---------------------------------------------------------
     iters = []
+    last = {}
 
     def step_dev(i):
         with torch.no_grad():
-            from_differential(M, us[i % R], "Cholesky")     # asynchronous: one persistent-kernel launch per solve
+            x = from_differential(M, us[i % R], "Cholesky")     # asynchronous: one persistent-kernel launch per solve
+        if i == args.steps - 1:
+            last["x"] = x
 
     ms_total, launches = timed(step_dev, args.steps, args.warmup)
+    x_last = last.pop("x").cpu()                                # what the last timed step returned (for --dump-outputs)
     for i in range(R):                                          # iteration counts per right-hand side (untimed)
         with torch.no_grad():
             from_differential(M, us[i], "Cholesky")
@@ -639,6 +646,10 @@ def run_b200(args, wl, wl_name):
             "extra": extra,
         }
         print(json.dumps(line))
+    if rank == 0 and args.dump_outputs:
+        # the solution (V, 3) of the last timed step, for output-for-output comparison of two builds on the same inputs
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "solution.npy"), x_last.numpy().astype(np.float32))
     if world > 1:
         dist.destroy_process_group()
     return 0
@@ -654,7 +665,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-spmv-4m", action="store_true", help="skip the 4M-vertex SpMV roofline measurement")
     ap.add_argument("--no-config4", action="store_true", help="skip the config-4 sub-record (8 x 250K meshes over the ranks)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the solution of the last one to DIR/solution.npy (float32, V x 3)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":

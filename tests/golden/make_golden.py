@@ -1,12 +1,11 @@
 #!/usr/bin/env python
-"""Generate tests/golden/*.npz by running the UNMODIFIED reference (/root/reference) on the CPU.
-
-Run in the builder container only (the GPU box has no /root/reference):
-    python tests/golden/make_golden.py
+"""Generate tests/golden/*.npz by running the UNMODIFIED reference (rgl-epfl/large-steps-pytorch) on the CPU.
+The tests only read the stored files; the reference is needed only to regenerate them:
+    LARGESTEPS_REF=<checkout of rgl-epfl/large-steps-pytorch> python tests/golden/make_golden.py
 
 How the reference is made to run here without a GPU / without cholespy (nothing is copied into the repo):
   * largesteps/geometry.py hard-codes device='cuda' (geometry.py:60,83,125).  Its source text is read
-    from /root/reference at run time, the literal "device='cuda'" is replaced by "device='cpu'" in memory,
+    from the checkout at run time, the literal "device='cuda'" is replaced by "device='cpu'" in memory,
     and the result is exec'd as module `largesteps.geometry`.
   * largesteps/solvers.py imports cholespy (solvers.py:3), which is not installable offline.  A stub module
     is registered in sys.modules so ConjugateGradientSolver / DifferentiableSolve / from_differential(method='CG')
@@ -21,7 +20,7 @@ import warnings
 import numpy as np
 import torch
 
-REF = "/root/reference"
+REF = os.environ.get("LARGESTEPS_REF", "")
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "..", "..", "large-steps-pytorch_b200"))
 from largesteps_b200 import workloads  # noqa: E402  (mesh generators only)
@@ -31,6 +30,8 @@ torch.set_num_threads(4)
 
 
 def load_reference():
+    if not os.path.isfile(os.path.join(REF, "largesteps", "geometry.py")):
+        sys.exit("set LARGESTEPS_REF to a checkout of rgl-epfl/large-steps-pytorch")
     chol = types.ModuleType("cholespy")
     chol.CholeskySolverF = object
     chol.MatrixType = types.SimpleNamespace(COO=0)
